@@ -21,6 +21,8 @@ A step = one pass of the hot path (one search tick) over one synthetic player po
 Launch: `python bench.py --gpus 1 --steps K --warmup W`, or under torchrun for N>1
 (one rank per GPU; ranks own disjoint rating groups — no data-path collective).
 `--impl reference` times the CPU restatement of the reference loop (oracle/).
+`--dump-outputs DIR` writes the results of the last timed tick of `value` as DIR/*.npy (see dump_outputs), so that
+two builds can be compared output for output on the same seeded pool.
 """
 import argparse
 import importlib
@@ -93,6 +95,53 @@ class ClockSampler:
         hi = [x for x in sm if x >= 0.5 * max(sm)] if sm else []
         return {"sm_mhz": statistics.median(hi) if hi else None, "sm_max_mhz": max(smax) if smax else None,
                 "samples": len(sm), "reasons": sorted(reasons)}
+
+
+DUMP_ROWS = 1 << 19  # rows kept per array: 2^19 x (4 + 1 + 2 + 1) float64 columns = 32 MiB in all
+
+
+def read_device_results(pkg, eng, st):
+    """Host copies of what the last mm_tick_device left in HBM: lobby headers and u64 member ids."""
+    import types
+
+    import numpy as np
+    import torch
+
+    def fetch(ptr, nbytes):
+        if nbytes == 0:
+            return np.empty(0, np.uint8)
+        buf = types.SimpleNamespace(__cuda_array_interface__={
+            "shape": (nbytes,), "typestr": "|u1", "data": (ptr, False), "version": 3})
+        return torch.as_tensor(buf, device="cuda").cpu().numpy()
+
+    d_lob, d_mem = eng.results_device()
+    return (fetch(d_lob, 8 * st.n_lobbies).view(pkg.engine.LOBBY_DTYPE),
+            fetch(d_mem, 8 * st.n_matched).view(np.uint64))
+
+
+def dump_outputs(out_dir, st, lob, mem):
+    """One tick's results as float64 .npy files with exact values: tick_counts (pool_before, n_lobbies, n_matched,
+    n_residual, n_dead), lobbies (first_member, n_members, mode, group), member_ids (high and low 32 bits).  An array
+    longer than DUMP_ROWS is a fixed seeded sample of its rows; <name>_rows holds their row numbers."""
+    import numpy as np
+
+    def rows(n):
+        if n <= DUMP_ROWS:
+            return np.arange(n)
+        return np.sort(np.random.default_rng(0).choice(n, DUMP_ROWS, replace=False))
+
+    r_lob, r_mem = rows(len(lob)), rows(len(mem))
+    sl, sm = lob[r_lob], mem[r_mem]
+    arrays = {
+        "tick_counts": np.array([st.pool_before, st.n_lobbies, st.n_matched, st.n_residual, st.n_dead], np.float64),
+        "lobbies": np.stack([sl["first_member"], sl["n_members"], sl["mode"], sl["group"]], axis=1).astype(np.float64),
+        "lobbies_rows": r_lob.astype(np.float64),
+        "member_ids": np.stack([sm >> np.uint64(32), sm & np.uint64(0xFFFFFFFF)], axis=1).astype(np.float64),
+        "member_ids_rows": r_mem.astype(np.float64),
+    }
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 def run_reference(args, rank, world):
@@ -182,6 +231,7 @@ def stream_leg(pkg, device, seconds, rate, dt_ms, groups=32, max_spread=-1):
 
 
 def main():
+    sys.dont_write_bytecode = True  # the tree may be read-only: bench.py writes nothing there
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
     ap.add_argument("--steps", type=int, default=20)
@@ -207,7 +257,12 @@ def main():
     ap.add_argument("--tick-impl", type=int, default=None, help="1 = one fused cooperative launch (default), 0 = four launches")
     ap.add_argument("--max-spread", type=int, default=None,
                     help="EXTENSION (policy S1, not the BASELINE workload): a lobby spans at most W rating points")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last timed tick of `value` returned (rank 0) as "
+                         "DIR/<name>.npy, float64, 32 MiB at most")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the GPU tick's results; --impl reference returns none")
 
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -253,8 +308,9 @@ def main():
 
     flush = torch.empty(256 << 20, dtype=torch.uint8, device="cuda")  # > 126 MB L2
 
-    def device_timed(cfg_, ids_, rating_, mode_, ts_, steps, warmup):
-        """K ticks of one resident pool (restored from a device snapshot, L2 flushed, both untimed)."""
+    def device_timed(cfg_, ids_, rating_, mode_, ts_, steps, warmup, read_results=False):
+        """K ticks of one resident pool (restored from a device snapshot, L2 flushed, both untimed); read_results:
+        also return host copies of the last tick's lobby headers and member ids (read after the timed region)."""
         eng = pkg.Engine(cfg_)
         options(eng)
         assert eng.enqueue(ids_, rating_, mode_, ts_).all()
@@ -277,14 +333,16 @@ def main():
             phases.append((st.hist_us, st.scan_us, st.place_us, st.epilogue_us))
         barrier()
         wall = time.perf_counter() - t0
+        results = read_device_results(pkg, eng, st) if read_results else None
         eng.close()
-        return sum(dev_us) * 1e-6, st, phases, wall
+        return sum(dev_us) * 1e-6, st, phases, wall, results
 
     # ---- weak leg (the contract's line): every rank holds a full-size pool of its own seed stream -------------
     ids, rating, mode, ts = pkg.synth.gen_pool(1, n, first=rank * n, mode=mode_idx)
     sampler = ClockSampler(local)
     sampler.start()
-    tick_s, st, phases, wall_s = device_timed(cfg, ids, rating, mode, ts, args.steps, args.warmup)
+    tick_s, st, phases, wall_s, last_results = device_timed(cfg, ids, rating, mode, ts, args.steps, args.warmup,
+                                                            read_results=bool(args.dump_outputs) and rank == 0)
     launches_per_tick = st.n_launches
     lobbies_per_step = st.n_lobbies
     if world > 1:
@@ -306,7 +364,7 @@ def main():
         mine = shard.route(cfg, g_rating, world) == rank  # the Generic stage's routing (generic/worker.ex:46-69)
         n_mine = int(mine.sum())
         s_steps = max(3, args.steps // 2)
-        s_tick, s_st, s_ph, _ = device_timed(cfg, g_ids[mine], g_rating[mine], g_mode[mine], g_ts[mine], s_steps, args.warmup)
+        s_tick, s_st, s_ph, _, _ = device_timed(cfg, g_ids[mine], g_rating[mine], g_mode[mine], g_ts[mine], s_steps, args.warmup)
         t = torch.tensor([s_tick], device="cuda", dtype=torch.float64)
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
         tl = torch.tensor([s_st.n_lobbies, n_mine], device="cuda", dtype=torch.int64)
@@ -557,6 +615,8 @@ def main():
             "cpu_baseline": cpu, "e2e": e2e, "strong": strong, "stream": stream,
             "gpu_launches": launches_per_tick * args.steps, "clocks": clocks,
         }
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, st, *last_results)
         print(json.dumps(line), flush=True)
     if world > 1:
         dist.destroy_process_group()
